@@ -4,8 +4,11 @@
   python bench.py --gpus 1 --steps 5 --warmup 3            # our arm (C2: medium, 32 x 256 phonemes)
   python bench.py --impl reference --steps 2 --warmup 1    # reference arm: CPU path on host cores
   torchrun ... bench.py --gpus N ...                        # one rank per GPU, weak scaling (32 utts / GPU)
+  python bench.py --steps 5 --warmup 3 --dump-outputs DIR  # also write the last timed step's waveforms to DIR
 
-A "step" is one pass of the phoneme-id -> waveform hot path over one batch of synthetic ids.
+A "step" is one pass of the phoneme-id -> waveform hot path over one batch of synthetic ids.  The ids, the voice and
+the noise (a per-voice call counter seeds it) depend only on the arguments, so two builds can be compared on the
+arrays --dump-outputs writes.  The synthetic voices are written to a temporary directory, never into the tree.
 `value`   : whole-job audio-s/s, device-resident result (N > 1: incl. the NCCL id broadcast / length all-reduce).
 `e2e`     : same metric, host ids in -> host waveforms out: `speak_batch_ids` (N = 1) / `shard.Frontend` (N > 1: one
             frontend on rank 0, results through a page-locked host segment shared by the ranks).
@@ -18,10 +21,13 @@ Prints ONE JSON line on rank 0.
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -35,6 +41,7 @@ sys.path.insert(0, ROOT)
 
 SR = 22050
 HOP = 256
+DUMP_BUDGET = 64_000_000        # bytes --dump-outputs may write in all
 
 
 def ncu_traffic():
@@ -45,6 +52,24 @@ def ncu_traffic():
         with open(p) as f:
             return json.load(f)
     return None
+
+
+def dump_outputs(out_dir: str, waves) -> None:
+    """The waveforms of one step as its caller receives them: `audio_000.npy`, ... (float32, one per utterance, in
+    batch order) and their lengths in samples (`samples.npy`, float64).  When the waveforms exceed DUMP_BUDGET together,
+    each is cut to the same fraction of its samples, at sorted positions drawn from a generator seeded with the
+    utterance's index: equal lengths give equal positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    lens = np.array([len(w) for w in waves], dtype=np.float64)
+    np.save(os.path.join(out_dir, "samples.npy"), lens)
+    room = DUMP_BUDGET - lens.nbytes - 256 * (len(waves) + 1)         # 256: bound on one .npy header
+    frac = min(1.0, room / (4.0 * max(lens.sum(), 1.0)))
+    for b, w in enumerate(waves):
+        w = np.asarray(w, dtype=np.float32)
+        if frac < 1.0:
+            pick = np.random.default_rng([20261017, b]).choice(len(w), int(len(w) * frac), replace=False)
+            w = w[np.sort(pick)]
+        np.save(os.path.join(out_dir, f"audio_{b:03d}.npy"), w)
 
 
 def read_peaks():
@@ -168,7 +193,11 @@ def main():
     ap.add_argument("--no-c5", action="store_true", help="skip the C5 mixed-length corpus")
     ap.add_argument("--c5-utts", type=int, default=1024)
     ap.add_argument("--no-secondary", action="store_true", help="skip the C1 / C3 secondary lines (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the waveforms of the last one to DIR as .npy (one process only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1 or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200, one process and --steps >= 1")
 
     from sonata_b200 import workload
     quality, B, NPH = workload.CONFIGS[args.workload]
@@ -227,12 +256,10 @@ def main():
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    if rank == 0:
-        for q_ in {quality, "medium", "high"}:
-            voicegen.write_voice(voicegen.default_voice_dir(), q_)
-    if world > 1:
-        dist.barrier()
-    cfg_path = voicegen.write_voice(voicegen.default_voice_dir(), quality)
+    # every process writes the (seeded, identical) voices into a directory of its own: the tree may be read-only
+    voice_dir = tempfile.mkdtemp(prefix="sonata_b200_voices_")
+    atexit.register(shutil.rmtree, voice_dir, True)
+    cfg_path = voicegen.write_voice(voice_dir, quality)
     model = sonata_b200.from_config_path(cfg_path, device=local_rank)
     model.set_backend(args.backend)
     lib = _native.lib()
@@ -271,21 +298,23 @@ def main():
             for k in ("ms", "flops", "bytes", "launches"):
                 acc[k] += r[k]
 
-    def step_device(record):
-        """device-resident pass (results stay in HBM); returns this rank's (audio seconds, device ms)"""
+    def step_device(record, keep=False):
+        """device-resident pass (results stay in HBM); returns this rank's (audio seconds, device ms) and, with `keep`
+        (N = 1), the job still holding its results, for the caller to close"""
         if fe is None:
             job = SynthesisJob(model, all_batches)
             ms = job.run()
             samples = job.lengths()[1]
             if record:
                 add_profile(job.profile())
-            job.close()
-            return sum(samples) / SR, ms
+            if not keep:
+                job.close()
+            return sum(samples) / SR, ms, (job if keep else None)
         fe.synthesize(all_batches if rank == 0 else None, device_only=True)
         owner, samples = fe.last_table
         if record:
             add_profile(fe.last_profile)
-        return float(samples[owner == rank].sum()) / SR, fe.last_device_ms
+        return float(samples[owner == rank].sum()) / SR, fe.last_device_ms, None
 
     def step_e2e():
         """host ids in -> host waveforms out, through the public call (N = 1) / the one-frontend path (N > 1); returns
@@ -307,14 +336,17 @@ def main():
     launches0 = int(lib.sb200_launch_count())
     sampler.mark()
     t0 = time.perf_counter()
-    audio_local, dev_ms = 0.0, 0.0
+    audio_local, dev_ms, last = 0.0, 0.0, None
     for s in range(args.steps):
-        a_, ms = step_device(True)
+        a_, ms, last = step_device(True, keep=bool(args.dump_outputs) and s == args.steps - 1)
         audio_local += a_; dev_ms += ms
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     launches = int(lib.sb200_launch_count()) - launches0
+    if last is not None:
+        dump_outputs(args.dump_outputs, [a.samples.as_slice() for a in last.fetch()])
+        last.close()
     wall_max, audio_total = reduce_pair(wall, audio_local)
     dev_ms_max, _ = reduce_pair(dev_ms, 0.0)
     value = audio_total / wall_max
@@ -383,7 +415,7 @@ def main():
         for name in ("C1", "C3"):
             q2, B2, N2 = workload.CONFIGS[name]
             m2 = model if q2 == quality else sonata_b200.from_config_path(
-                voicegen.write_voice(voicegen.default_voice_dir(), q2), device=local_rank)
+                voicegen.write_voice(voice_dir, q2), device=local_rank)
             m2.set_backend(args.backend)
             bt = [workload.synthetic_ids(N2, utt=u) for u in range(B2)]
             steps2 = 30 if name == "C1" else 4

@@ -4,6 +4,7 @@ payloads, fp16 tensors, packed and unpacked dims, and the failure modes it must 
 import json
 import os
 import struct
+import zlib
 
 import numpy as np
 import pytest
@@ -134,16 +135,24 @@ def test_multi_speaker_import_and_garbage(tmp_path):
         onnx_import.read_initializers(str(bad))
 
 
-REAL_ONNX = "/root/reference/deps/libtashkeel/crates/core/data/ort/model.onnx"
+GOLDEN_ONNX = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "onnx")
+REAL_ONNX = os.path.join(GOLDEN_ONNX, "libtashkeel_sample.onnx")
 
 
-@pytest.mark.skipif(not os.path.exists(REAL_ONNX), reason="the reference checkout (build container only) holds the file")
 def test_reader_parses_a_real_exported_onnx_file():
-    """Every other test here reads files written by this suite's own writer.  The one ONNX file a real exporter produced
-    that exists offline is the libtashkeel model vendored by the reference (a torch.onnx export, not a Piper voice): the
-    hand-rolled protobuf reader must get its initialisers out -- names, dims, dtypes, raw payloads -- and account for
-    nearly all of the file's bytes."""
+    """Every other test here reads files written by this suite's own writer.  This one reads what a real exporter
+    produced: libtashkeel's model (a torch.onnx export, not a Piper voice), shrunk to a sample that keeps the exporter's
+    encoding of every initialiser (tests/golden/onnx/make_onnx_golden.py).  The hand-rolled protobuf reader must get the
+    initialisers out -- names, dims, dtypes, raw payloads, as the manifest written alongside the sample lists them --
+    and account for nearly all of the file's bytes."""
+    with open(os.path.join(GOLDEN_ONNX, "libtashkeel_sample.json")) as f:
+        manifest = json.load(f)["initializers"]
     t = onnx_import.read_initializers(REAL_ONNX)
+    assert list(t) == [e["name"] for e in manifest]
+    for e in manifest:
+        a = t[e["name"]]
+        assert e["data_type"] == 1 and a.dtype == np.float32 and list(a.shape) == e["dims"], e["name"]
+        assert zlib.crc32(np.ascontiguousarray(a).astype("<f4").tobytes()) == e["crc32"], e["name"]
     assert len(t) == 127
     assert t["char_emb.weight"].shape == (54, 56) and t["char_emb.weight"].dtype == np.float32
     assert t["attn_layers.0.ccm.batchnorm.running_var"].shape == (112,)
